@@ -20,6 +20,8 @@ died out (12 033 server messages per value on the 64x64 grid, BASELINE.md).
 --config selects the other BASELINE configs at full size: broadcast-lat1 (constant 1 ms latency:
 the timing wheel is on), gset16k (configs[2]), raft64k (configs[3]), txn256k (configs[4]).
 --verify adds a sharded parity run (256 nodes x 2000 values: merged journal digest vs the oracle).
+--dump-outputs DIR writes what the timed steps computed (counters, clock, state of a seeded sample of
+nodes; see dump_outputs) as .npy files, so that two builds can be compared output for output.
 --impl reference times the CPU restatement instead (the JVM reference cannot run on this box: no
 java/lein), on all host cores as independent replicas fed by one persistent worker pool.
 """
@@ -103,6 +105,11 @@ class Workload:
     def between_steps(self, sim, step):
         """nemesis hook, called before step `step` runs (same on every rank)"""
 
+    def dump_values(self, step):
+        """--dump-outputs: the values whose presence in the sampled nodes' seen sets is written after step
+        `step` (None: the workload keeps no seen sets)"""
+        return None
+
     def alg_bytes(self, sends, recvs):
         return ALG_SEND_B * sends + (ALG_RECV_B + self.extra_recv_bytes) * recvs
 
@@ -159,6 +166,10 @@ class Broadcast(Workload):
         ops["body"]["msg_id"] = (g // np.uint64(self.n_clients) + np.uint64(1)).astype(np.uint32)
         ops["body"]["p0"] = g.astype(np.uint32)
         return ops
+
+    def dump_values(self, step):
+        first = step * self.step_ticks * self.V          # the values injected by this step
+        return np.arange(first, first + self.step_ticks * self.V, dtype=np.uint64)
 
     def config_extra(self):
         return {"latency": "constant %d ms" % self.latency_ms, "values_per_tick": self.V,
@@ -238,6 +249,9 @@ class GSet16k(Workload):
         ops["body"]["msg_id"] = (np.uint64(1 << 20) + g // np.uint64(self.n_clients)).astype(np.uint32)
         ops["body"]["p0"] = (g % np.uint64(self.n_values)).astype(np.uint32)
         return ops
+
+    def dump_values(self, step):
+        return np.arange(self.n_values, dtype=np.uint64)
 
     def config_extra(self):
         return {"latency": "exponential, mean 100 ms", "p_loss": 0.1, "interval_ms": self.interval_ms,
@@ -638,6 +652,51 @@ def metric_name(wl):
     return "simulated msgs/sec (%s)" % wl.name
 
 
+# --------------------------------------------------------------------------- outputs
+DUMP_NODES = 128                 # seeded sample of nodes whose state --dump-outputs writes
+DUMP_VALUES = 32768              # at most this many values (seeded sample) per node: seen.npy stays <= 16 MB
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, sim, wl, step):
+    """--dump-outputs: what the timed path has computed once its last step (`step`) is done, as .npy files:
+    stats.npy     send / recv / msg counts of all endpoints, clients, servers (Sim.stats order), float64
+    clock.npy     virtual time (ns) and round, float64
+    net.npy       messages lost, messages dropped by partitions, replies to clients, float64
+    nodes.npy     the sampled node indices, float64
+    seen.npy      seen-set workloads: [node, value] = 1.0 where the sampled node holds the value, float32;
+    values.npy    its columns: the values the last step injected (g-set: every element), float64
+    raft.npy      Raft workload: Sim.raft_state of each sampled node (Sim.RAFT_FIELDS order), float64
+    The node and value samples are drawn from a fixed seed, so equal arguments give comparable files."""
+    from maelstrom_b200.engine import Sim, WORKLOADS
+    rng = np.random.default_rng(SEED)
+    nodes = np.sort(rng.choice(wl.n_nodes, size=min(DUMP_NODES, wl.n_nodes), replace=False))
+    st = sim.stats()
+    c = sim.counters()
+    out = {"stats": np.array([st[g][k] for g in ("all", "clients", "servers") for k in ("send-count", "recv-count", "msg-count")],
+                             dtype=np.float64),
+           "clock": np.array([sim.now, sim.round], dtype=np.float64),
+           "net": np.array([c["lost"], c["partition_drops"], sim.client_replies()], dtype=np.float64),
+           "nodes": nodes.astype(np.float64)}
+    values = wl.dump_values(step)
+    if values is not None:
+        if len(values) > DUMP_VALUES:
+            values = np.sort(rng.choice(values, size=DUMP_VALUES, replace=False))
+        out["values"] = values.astype(np.float64)
+        seen = np.zeros((len(nodes), len(values)), dtype=np.float32)
+        for i, k in enumerate(nodes):
+            held = np.zeros(sim.cfg.n_values, dtype=bool)
+            held[sim.node_set(int(k))] = True
+            seen[i] = held[values]
+        out["seen"] = seen
+    if sim.workload == WORKLOADS["lin-kv"]:
+        out["raft"] = np.array([[sim.raft_state(int(k))[f] for f in Sim.RAFT_FIELDS] for k in nodes], dtype=np.float64)
+    assert sum(a.nbytes for a in out.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------- GPU arm
 def make_sim(mb, wl, n_steps, journal_discard, device, world):
     kw = wl.sim_kwargs(n_steps, journal_discard)
@@ -771,6 +830,8 @@ def gpu_arm(args, rank, world, local_rank):
     torch.cuda.synchronize()
     after = lstats()
     c_after = sim.counters()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sim, wl, R + W + K - 1)
     if args.phase_cycles and world == 1:
         pc = sim.phase_cycles(False)
         names = ["fetch", "load+seen (PA)", "order (PB)", "first-sight+counts (PC)", "scan", "claims (PD)", "records+emissions (PE)",
@@ -954,10 +1015,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--phase-cycles", action="store_true", help="diagnostic: per-phase cycles per ticket on stderr; needs a -DMS_PHASE_TIMING build (MS_B200_LIB=...); not a bench run")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed steps computed into DIR/<name>.npy (one GPU)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the GPU path on one GPU")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

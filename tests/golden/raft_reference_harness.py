@@ -1,4 +1,4 @@
-"""Runs the reference's own Raft node, /root/reference/demo/python/raft.py, UNMODIFIED, as a
+"""Runs the reference's own Raft node, demo/python/raft.py of jepsen-io/maelstrom, UNMODIFIED, as a
 cluster inside this process and records every message it sends -- the trace the oracle's
 restatement (oracle/oracle.cpp node_raft / raft_actions) is pinned to.
 
@@ -14,8 +14,10 @@ and `random.random()` the k-th Philox draw of the node's step (the oracle's raft
 exact rationals so that the reference's comparisons are made without float rounding; messages get
 ids in emission order and are delivered in id order in the next round (latency 0, no loss).
 
-Needs /root/reference (build container only); the trace it produces is committed as
-tests/golden/raft_reference_trace.json (python tests/golden/raft_reference_harness.py).
+Needs a checkout of jepsen-io/maelstrom; what it produces is committed under tests/golden/
+(python tests/golden/raft_reference_harness.py <maelstrom checkout>): raft_reference_trace.json,
+raft_reference_trace_partition.json and raft_reference_trace_random.json (the random scenarios of
+random_raft_scenario for seeds RANDOM_SEEDS).
 """
 import json
 import os
@@ -23,10 +25,13 @@ import sys
 import types
 from fractions import Fraction
 
+import numpy as np
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
-RAFT_PY = "/root/reference/demo/python/raft.py"
+RAFT_PY = None                                                       # set by main()
 SEED = 0x4D41454C
+RANDOM_SEEDS = range(8)
 
 
 class Node:
@@ -192,6 +197,56 @@ def run(n, ops, events, until):
     return c
 
 
+def random_raft_scenario(seed):
+    """(n, ops, events, until_ms): random cluster size, client traffic (with a second `init` now and
+    then) and bulk partitions that come, change and sometimes heal."""
+    rng = np.random.default_rng(seed)
+    n = int(rng.integers(1, 6))
+    ops = [(0, "c%d" % i, "n%d" % i, {"type": "init", "msg_id": 1, "node_id": "n%d" % i,
+                                      "node_ids": ["n%d" % k for k in range(n)]}) for i in range(n)]
+    until = int(rng.integers(5000, 12000))
+    k = 1
+    times = sorted(int(t) for t in rng.integers(0, until, size=int(rng.integers(5, 60))))
+    for t in times:
+        k += 1
+        dest = int(rng.integers(n))
+        kind = int(rng.integers(4))
+        body = {"msg_id": k, "key": int(rng.integers(3))}
+        if kind == 0:
+            body.update(type="read")
+        elif kind == 1:
+            body.update(type="write", value=int(rng.integers(5)))
+        elif kind == 2:
+            body.update({"type": "cas", "from": int(rng.integers(5)), "to": int(rng.integers(5))})
+        else:
+            body = {"msg_id": k, "type": "init", "node_id": "n%d" % dest, "node_ids": []}    # "Can't init twice!"
+        ops.append((t, "c%d" % int(rng.integers(n)), "n%d" % dest, body))
+    events = []
+    for t in sorted(int(t) for t in rng.integers(2000, until, size=int(rng.integers(0, 5)))):
+        events.append((t, "heal" if rng.integers(3) == 0 else [int(x) for x in rng.integers(0, 2, size=n)]))
+    return n, ops, events, until
+
+
+def run_random(n, ops, events, until):
+    """A random_raft_scenario on the reference: bulk partitions with arbitrary sides, repeated, healed or
+    not.  None when virtual time freezes: some next_index went non-positive, replicate_log now raises
+    before it records the replication and so replicates again in every loop iteration; at latency 0
+    that freezes virtual time (DESIGN.md 2.3).  The oracle gives up the same way (or_run)."""
+    c = Cluster(n)
+    i = j = 0
+    while c.now_ns < until * 1_000_000:
+        while j < len(events) and events[j][0] * 1_000_000 <= c.now_ns:
+            c.component = None if events[j][1] == "heal" else list(events[j][1])
+            j += 1
+        while i < len(ops) and ops[i][0] * 1_000_000 <= c.now_ns:
+            c.client_send(ops[i][1], ops[i][2], ops[i][3])
+            i += 1
+        c.run_round()
+        if c.round > until + 30_000:
+            return None
+    return c
+
+
 def canonical(m, n):
     """One sent message as a flat tuple: (id, time_ms, src, dest, type, fields...); endpoints as the
     engine numbers them (servers 0..n-1, then clients)."""
@@ -241,13 +296,36 @@ def dump(c, n, until, name, extra=None):
     print(name, "messages", len(c.trace), "rounds", c.round, "final", [(x["state"], x["term"], x["log_size"]) for x in states])
 
 
-def main():
+def dump_random(name):
+    with open(os.path.join(HERE, name), "w") as f:                      # one message per line
+        f.write('{"reference": "demo/python/raft.py", "seed": %d, "scenarios": [\n' % SEED)
+        for k, seed in enumerate(RANDOM_SEEDS):
+            n, ops, events, until = random_raft_scenario(seed)
+            c = run_random(n, ops, events, until)
+            assert c is not None, "seed %d freezes virtual time: pick other seeds" % seed
+            final = [{"state": nd.raft.state, "term": nd.raft.current_term, "commit_index": nd.raft.commit_index,
+                      "log_size": nd.raft.log.size(), "last_applied": nd.raft.last_applied} for nd in c.nodes]
+            head = {"scenario_seed": seed, "n": n, "until_ms": until, "rounds": c.round, "final": final}
+            f.write(",\n" if k else "")
+            f.write(json.dumps(head, sort_keys=True)[:-1] + ', "messages": [\n')
+            f.write(",\n".join(json.dumps(canonical(m, n)) for m in c.trace))
+            f.write("\n]}")
+            print(name, "seed", seed, "messages", len(c.trace), "rounds", c.round)
+        f.write("\n]}\n")
+
+
+def main(maelstrom_checkout):
+    global RAFT_PY
+    RAFT_PY = os.path.join(maelstrom_checkout, "demo", "python", "raft.py")
     n = 3
     ops, until = scenario(None, n)
     dump(run(n, ops, [], until), n, until, "raft_reference_trace.json")
     ops, events, until = partition_scenario(5)
     dump(run(5, ops, events, until), 5, until, "raft_reference_trace_partition.json", {"events": events})
+    dump_random("raft_reference_trace_random.json")
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/raft_reference_harness.py <jepsen-io/maelstrom checkout>")
+    main(sys.argv[1])

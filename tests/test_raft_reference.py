@@ -1,10 +1,11 @@
 """Pins the oracle's Raft restatement to the reference's own code.  tests/golden/
 raft_reference_trace.json is every message sent by a 3-node cluster of the UNMODIFIED
-/root/reference/demo/python/raft.py, executed by tests/golden/raft_reference_harness.py under the
+demo/python/raft.py of jepsen-io/maelstrom, executed by tests/golden/raft_reference_harness.py under the
 schedule of DESIGN.md section 2.8 (virtual clock, Philox draws).  The oracle, given the same
 client operations, must send the same messages with the same ids at the same times, and end in
-the same node states.  Where /root/reference is mounted the fixture is also regenerated and
-compared, so it cannot drift from the reference."""
+the same node states.  raft_reference_trace_partition.json and raft_reference_trace_random.json hold the
+same for a partitioned 5-node cluster and for random scenarios; the harness regenerates all three
+from a maelstrom checkout."""
 import json
 import os
 import sys
@@ -129,50 +130,6 @@ def test_oracle_matches_the_reference_through_a_partition():
     assert any(w[4] == "append_entries_res" and w[6] == 0 for w in want)     # a follower rejected an append
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/demo/python/raft.py"),
-                    reason="the reference tree is only mounted in the build container")
-def test_fixtures_are_what_the_reference_produces():
-    import raft_reference_harness as H
-    fix = json.load(open(FIXTURE))
-    ops, until = H.scenario(None, fix["n"])
-    c = H.run(fix["n"], ops, [], until)
-    assert [H.canonical(m, fix["n"]) for m in c.trace] == fix["messages"] and c.round == fix["rounds"]
-    fix = json.load(open(FIXTURE.replace(".json", "_partition.json")))
-    ops, events, until = H.partition_scenario(fix["n"])
-    c = H.run(fix["n"], ops, events, until)
-    assert [H.canonical(m, fix["n"]) for m in c.trace] == fix["messages"] and c.round == fix["rounds"]
-
-
-def random_raft_scenario(seed):
-    """(n, ops, events, until_ms): random cluster size, client traffic (with a second `init` now and
-    then) and bulk partitions that come, change and sometimes heal."""
-    rng = np.random.default_rng(seed)
-    n = int(rng.integers(1, 6))
-    ops = [(0, "c%d" % i, "n%d" % i, {"type": "init", "msg_id": 1, "node_id": "n%d" % i,
-                                      "node_ids": ["n%d" % k for k in range(n)]}) for i in range(n)]
-    until = int(rng.integers(5000, 12000))
-    k = 1
-    times = sorted(int(t) for t in rng.integers(0, until, size=int(rng.integers(5, 60))))
-    for t in times:
-        k += 1
-        dest = int(rng.integers(n))
-        kind = int(rng.integers(4))
-        body = {"msg_id": k, "key": int(rng.integers(3))}
-        if kind == 0:
-            body.update(type="read")
-        elif kind == 1:
-            body.update(type="write", value=int(rng.integers(5)))
-        elif kind == 2:
-            body.update({"type": "cas", "from": int(rng.integers(5)), "to": int(rng.integers(5))})
-        else:
-            body = {"msg_id": k, "type": "init", "node_id": "n%d" % dest, "node_ids": []}    # "Can't init twice!"
-        ops.append((t, "c%d" % int(rng.integers(n)), "n%d" % dest, body))
-    events = []
-    for t in sorted(int(t) for t in rng.integers(2000, until, size=int(rng.integers(0, 5)))):
-        events.append((t, "heal" if rng.integers(3) == 0 else [int(x) for x in rng.integers(0, 2, size=n)]))
-    return n, ops, events, until
-
-
 def oracle_for(n, ops, seed):
     s = O.Sim(n, workload=O.W_RAFT, seed=seed)
     clients = [s.add_endpoint("c%d" % q) for q in range(n)]
@@ -208,44 +165,26 @@ def test_frozen_virtual_time_is_reported_not_spun_on():
     # seed 132 of the scenario generator drives a next_index non-positive: the reference's
     # replicate_log then raises before recording the replication and replicates again in every loop
     # iteration -- at latency 0 a message is always due "now" and virtual time stops (DESIGN.md 2.3)
-    n, ops, events, until = random_raft_scenario(132)
+    import raft_reference_harness as H
+    n, ops, events, until = H.random_raft_scenario(132)
     s = oracle_for(n, ops, 0x4D41454C)
     with pytest.raises(RuntimeError, match="not advancing"):
         run_events(s, events, until)
     assert s.now < until * 1_000_000
 
 
-def fuzz_seeds():
-    a, b = (int(x) for x in os.environ.get("MS_FUZZ_RAFTREF_SEEDS", "0:2").split(":"))
-    return list(range(a, b))
+RANDOM = {r["scenario_seed"]: r for r in json.load(open(FIXTURE.replace(".json", "_random.json")))["scenarios"]}
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/demo/python/raft.py"),
-                    reason="the reference tree is only mounted in the build container")
-@pytest.mark.parametrize("seed", fuzz_seeds())
+@pytest.mark.parametrize("seed", sorted(RANDOM))
 def test_random_scenarios_against_the_executed_reference(seed):
     # random cluster size, client traffic and partitions (arbitrary sides, repeated, healed or not):
-    # the reference's raft.py under the harness and the oracle must send the same messages
+    # the oracle must send the messages the reference's raft.py sent under the harness
     import raft_reference_harness as H
-    n, ops, events, until = random_raft_scenario(seed)
-
-    # reference
-    c = H.Cluster(n)
-    i = j = 0
-    while c.now_ns < until * 1_000_000:
-        while j < len(events) and events[j][0] * 1_000_000 <= c.now_ns:
-            c.component = None if events[j][1] == "heal" else list(events[j][1])
-            j += 1
-        while i < len(ops) and ops[i][0] * 1_000_000 <= c.now_ns:
-            c.client_send(ops[i][1], ops[i][2], ops[i][3])
-            i += 1
-        c.run_round()
-        if c.round > until + 30_000:
-            # Zeno: some next_index went non-positive, replicate_log now raises before it records the
-            # replication and so replicates again in every loop iteration; at latency 0 that freezes
-            # virtual time (DESIGN.md 2.3).  The oracle gives up the same way (or_run).
-            pytest.skip("the reference spins at a frozen instant in this scenario")
-    want = [tuple(H.canonical(m, n)) for m in c.trace]
+    n, ops, events, until = H.random_raft_scenario(seed)
+    fix = RANDOM[seed]
+    assert (n, until) == (fix["n"], fix["until_ms"])
+    want = [tuple(m) for m in fix["messages"]]
 
     s = oracle_for(n, ops, H.SEED)
     run_events(s, events, until)
@@ -253,9 +192,9 @@ def test_random_scenarios_against_the_executed_reference(seed):
     got = canonical_from_oracle(s, ev, bd)
     for g, w in zip(got, want):
         assert g == w, (g, w)
-    assert len(got) == len(want) and s.round == c.round
+    assert len(got) == len(want) and s.round == fix["rounds"]
     code = {"nascent": 0, "follower": 1, "candidate": 2, "leader": 3}
-    for q, nd in enumerate(c.nodes):
+    for q, nd in enumerate(fix["final"]):
         st = s.raft_state(q)
         assert (st["state"], st["term"], st["commit_index"], st["log_size"], st["last_applied"]) == \
-            (code[nd.raft.state], nd.raft.current_term, nd.raft.commit_index, nd.raft.log.size(), nd.raft.last_applied)
+            (code[nd["state"]], nd["term"], nd["commit_index"], nd["log_size"], nd["last_applied"])
