@@ -112,7 +112,9 @@ struct Params {
   uint32_t* limit;           // snapshot of tail at the start of the round
   uint32_t* head;            // previous snapshot: window is [head, limit)
   uint64_t* ep_born;         // next-message-id when the endpoint slot was (re)registered: wheel records with a smaller id are not for it
-  uint4*    ring;            // 48-B records (3 vectors): n_servers rings of ring_cap_s, then rings of ring_cap
+  uint4*    ring;            // 48-B records in two planes (DESIGN.md 3.1): ring_slots 16-B order keys, then
+                             // ring_slots 32-B bodies; slots: n_servers rings of ring_cap_s, then rings of ring_cap
+  uint64_t  ring_slots;      // slots of all rings together (equal on every shard)
   uint32_t  ring_cap, ring_cap_s;      // per endpoint: others / servers (powers of two)
   uint32_t  n_ep, n_servers, n_inj_tickets, max_window, max_window_s;
   // per-round history (ring of `hist` rows, stride t_max entries)

@@ -631,7 +631,8 @@ static int build_sim(ms_sim* s, const ms_config* in) {
   if ((rc = s->dalloc(&P.ep_born, M))) return rc;
   {
     void* ptr = nullptr;
-    CK(cudaMalloc(&ptr, ((size_t)c.n_nodes * c.server_ring_cap + (size_t)(M - c.n_nodes) * c.ring_cap) * 48));
+    P.ring_slots = (size_t)c.n_nodes * c.server_ring_cap + (size_t)(M - c.n_nodes) * c.ring_cap;
+    CK(cudaMalloc(&ptr, P.ring_slots * 48));   // key plane (16 B per slot), then body plane (32 B per slot)
     s->allocs.push_back(ptr);
     P.ring = (uint4*)ptr;
   }
@@ -1875,6 +1876,7 @@ struct ShardBlob {   // MS_SHARD_BLOB_BYTES
   uint32_t max_endpoints, ring_cap, hist, pad;
   cudaIpcMemHandle_t ring, tail, head, rt_cnt, bar;
   cudaIpcMemHandle_t gs_snap, gs_tag;   // pad = 1: g-set snapshot rows, tags; pad = 2: Raft payload heap, handle table
+  uint64_t ring_slots;                  // a peer's body plane starts ring_slots vectors into its ring
 };
 static_assert(sizeof(ShardBlob) <= MS_SHARD_BLOB_BYTES, "blob too large");
 
@@ -1886,6 +1888,7 @@ int ms_shard_handles(ms_sim* s, void* blob_out) {
   b.magic = 0x4253534Du;
   b.shard_id = s->P.shard_id; b.n_shards = s->P.n_shards; b.t_max = s->P.t_max;
   b.max_endpoints = s->cfg.max_endpoints; b.ring_cap = s->P.ring_cap ^ (s->P.ring_cap_s << 1); b.hist = s->P.hist;
+  b.ring_slots = s->P.ring_slots;
   CK(cudaIpcGetMemHandle(&b.ring, s->P.ring));
   CK(cudaIpcGetMemHandle(&b.tail, s->P.tail));
   CK(cudaIpcGetMemHandle(&b.head, s->P.head));
@@ -1912,7 +1915,7 @@ int ms_shard_connect(ms_sim* s, uint32_t peer, const void* blob) {
   memcpy(&b, blob, sizeof b);
   if (b.magic != 0x4253534Du || b.shard_id != peer || peer >= s->P.n_shards || b.n_shards != s->P.n_shards ||
       b.t_max != s->P.t_max || b.max_endpoints != s->cfg.max_endpoints || b.ring_cap != (s->P.ring_cap ^ (s->P.ring_cap_s << 1)) ||
-      b.hist != s->P.hist) {
+      b.hist != s->P.hist || b.ring_slots != s->P.ring_slots) {
     set_err("ms_shard_connect: peer blob does not match this simulation's configuration");
     return MS_ERR_ARG;
   }

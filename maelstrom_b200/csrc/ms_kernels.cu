@@ -108,7 +108,7 @@ __device__ __forceinline__ bool round_skipped(const Params& p, const DevState* s
 __device__ __forceinline__ uint32_t slot_tag(uint64_t round) { return 0x80000000u | (uint32_t)(round & 0x7FFFFFFFull); }
 
 // ------------------------------------------------------------------ ring records
-// 48-B inbox record: v0 = order key {idx, ticket, round}, v1 = {src, dest,
+// 48-B record: v0 = order key {idx, ticket, round}, v1 = {src, dest,
 // msg_id, in_reply_to}, v2 = {type | flags << 16, p0, p1}.
 struct Rec {
   uint64_t round;
@@ -119,10 +119,16 @@ struct Rec {
   uint64_t p1;
 };
 
+__device__ __forceinline__ void rec_pack(const Rec& r, uint4& a, uint4& b, uint4& c) {
+  a = make_uint4(r.idx, r.ticket, (uint32_t)r.round, (uint32_t)(r.round >> 32));
+  b = make_uint4(r.src, r.dest, r.msg_id, r.in_reply_to);
+  c = make_uint4(r.tf, r.p0, (uint32_t)r.p1, (uint32_t)(r.p1 >> 32));
+}
+// timing-wheel slot: the three vectors side by side
 __device__ __forceinline__ void rec_store(uint4* slot, const Rec& r) {
-  st_v4(slot + 0, make_uint4(r.idx, r.ticket, (uint32_t)r.round, (uint32_t)(r.round >> 32)));
-  st_v4(slot + 1, make_uint4(r.src, r.dest, r.msg_id, r.in_reply_to));
-  st_v4(slot + 2, make_uint4(r.tf, r.p0, (uint32_t)r.p1, (uint32_t)(r.p1 >> 32)));
+  uint4 a, b, c;
+  rec_pack(r, a, b, c);
+  st_v4(slot + 0, a); st_v4(slot + 1, b); st_v4(slot + 2, c);
 }
 __device__ __forceinline__ Rec rec_unpack(uint4 a, uint4 b, uint4 c) {
   Rec r;
@@ -141,8 +147,52 @@ __device__ __forceinline__ size_t ring_base(const Params& p, uint32_t e) {
   return e < p.n_servers ? (size_t)e * p.ring_cap_s
                          : (size_t)p.n_servers * p.ring_cap_s + (size_t)(e - p.n_servers) * p.ring_cap;
 }
-__device__ __forceinline__ uint4* ring_slot(const Params& p, uint4* ring, uint32_t e, uint32_t pos) {
-  return ring + (ring_base(p, e) + (pos & (ring_cap_of(p, e) - 1u))) * 3;
+// Slot g of the rings: order key v0 at ring[g] (key plane), v1 and v2 at ring[ring_slots + 2g] (body plane).
+// A window's keys are one contiguous run, so a reader that needs only the keys touches 16 B per message.
+__device__ __forceinline__ size_t ring_index(const Params& p, uint32_t e, uint32_t pos) {
+  return ring_base(p, e) + (pos & (ring_cap_of(p, e) - 1u));
+}
+__device__ __forceinline__ void ring_put(const Params& p, uint4* ring, size_t g, uint4 a, uint4 b, uint4 c) {
+  uint4* body = ring + p.ring_slots + 2 * g;
+  st_v4(ring + g, a); st_v4(body, b); st_v4(body + 1, c);
+}
+__device__ __forceinline__ void ring_store(const Params& p, uint4* ring, uint32_t e, uint32_t pos, const Rec& r) {
+  uint4 a, b, c;
+  rec_pack(r, a, b, c);
+  ring_put(p, ring, ring_index(p, e, pos), a, b, c);
+}
+// Compact record: server -> neighbor gossip written by k_round's fast path is the key vector alone,
+// {idx, ticket | kCompact, (uint32_t)round, value}; its body-plane slot is not written (it may hold a
+// stale record of an earlier lap).  The rest is implied: src = ticket - n_inj_tickets, dest = the
+// ring's owner, msg_id = in_reply_to = p1 = 0, tf = MS_T_BROADCAST.  Tickets fit in 24 bits
+// (kResolvedTicket), so the flag never collides with one; every ticket read from a key is masked.
+constexpr uint32_t kCompact = 1u << 31;
+__device__ __forceinline__ void ring_store_gossip(uint4* ring, size_t g, uint32_t idx, uint32_t ticket, uint64_t round,
+                                                  uint32_t value) {
+  st_v4(ring + g, make_uint4(idx, ticket | kCompact, (uint32_t)round, value));
+}
+// The round a compact key was sent in: its low word is stored, and it lies fewer than `hist` rounds
+// before the reader's round `cur`.
+__device__ __forceinline__ uint64_t compact_round(uint64_t cur, uint32_t lo) { return cur - (uint32_t)((uint32_t)cur - lo); }
+__device__ __forceinline__ Rec ring_expand(const Params& p, uint4 a, uint4 b, uint4 c, uint64_t cur, uint32_t owner) {
+  if (!(a.y & kCompact)) return rec_unpack(a, b, c);
+  Rec r;
+  r.idx = a.x; r.ticket = a.y & 0xFFFFFFu;
+  r.round = compact_round(cur, a.z);
+  r.src = r.ticket - p.n_inj_tickets; r.dest = owner; r.msg_id = 0; r.in_reply_to = 0;
+  r.tf = MS_T_BROADCAST; r.p0 = a.w; r.p1 = 0;
+  return r;
+}
+// Full record of slot g of `owner`'s ring as seen in round `cur`; key and body are loaded together.
+__device__ __forceinline__ Rec ring_load(const Params& p, const uint4* ring, size_t g, uint64_t cur, uint32_t owner) {
+  const uint4* body = ring + p.ring_slots + 2 * g;
+  return ring_expand(p, ring[g], body[0], body[1], cur, owner);
+}
+// The record of slot g without its order key, for a ring that never holds compact records (only a
+// broadcast server's ring does): one fewer load on the reply paths of clients, services and Raft.
+__device__ __forceinline__ Rec ring_load_body(const Params& p, const uint4* ring, size_t g) {
+  const uint4* body = ring + p.ring_slots + 2 * g;
+  return rec_unpack(make_uint4(0u, 0u, 0u, 0u), body[0], body[1]);
 }
 
 // dense id of (round, ticket, idx): id_base[round] + emit_prefix[round][ticket] + idx
@@ -343,8 +393,7 @@ __device__ __forceinline__ void emit_one(const Params& p, DevState* st, const Ne
     } else if (lat == 0) {                                           // deadline == now: next delta round
       cx.c_zero++;
       if (has_direct) {
-        uint4* ring_o = p.ring_sh[owner_of(r.dest, p.n_servers, p.n_shards)];
-        rec_store(ring_slot(p, ring_o, r.dest, direct_pos), r);
+        ring_store(p, p.ring_sh[owner_of(r.dest, p.n_servers, p.n_shards)], r.dest, direct_pos, r);
       } else {
         push = true;
       }
@@ -378,7 +427,7 @@ __device__ __forceinline__ void emit_one(const Params& p, DevState* st, const Ne
     if ((uint32_t)(pos - p.head_sh[o][r.dest]) >= ring_cap_of(p, r.dest)) {
       latch_error(st, E_RING_OVERFLOW, r.dest);
     } else {
-      rec_store(ring_slot(p, p.ring_sh[o], r.dest, pos), r);
+      ring_store(p, p.ring_sh[o], r.dest, pos, r);
     }
   }
 }
@@ -408,23 +457,22 @@ __device__ __forceinline__ bool gen_timer_due(const Params& p, const GenDev& g, 
 
 // One step of client e: its due replies in id order, then the timeout, then at most one invocation.
 // Returns true and fills `out` when the step sends a request.
-__device__ bool gen_step(const Params& p, DevState* st, uint32_t e, int64_t now, uint64_t round, const uint4* myring,
+__device__ bool gen_step(const Params& p, DevState* st, uint32_t e, int64_t now, uint64_t round, size_t my0,
                          uint32_t head, uint32_t my_mask, uint32_t n, const uint16_t* ord, const uint32_t* vals, Rec& out) {
   GenDev g = p.gc[e];
   for (uint32_t pos = 0; pos < n; pos++) {
     const uint32_t i = ord[pos];
     if (!(vals[i] & (1u << 30))) continue;                                 // V_RECV: cut by a partition
-    const uint4* rp = myring + (size_t)((head + i) & my_mask) * 3;
-    const uint4 vb = rp[1], vc = rp[2];
-    const uint32_t type = vc.x & 0xFFFFu, flags = vc.x >> 16;
-    if (!g.waiting_for || !(flags & MS_F_REPLY) || vb.w != g.waiting_for) continue;   // client.clj:106-107
+    const Rec m = ring_load_body(p, p.ring, my0 + ((head + i) & my_mask));
+    const uint32_t type = m.tf & 0xFFFFu, flags = m.tf >> 16;
+    if (!g.waiting_for || !(flags & MS_F_REPLY) || m.in_reply_to != g.waiting_for) continue;   // client.clj:106-107
     uint32_t outcome = MS_H_OK, err = 0, value = g.cur_value;
     if (type == MS_T_ERROR) {                                              // client.clj:165-172, errors.edn
-      err = vc.y;
+      err = m.p0;
       const bool definite = err != 0 && err != 13;
       outcome = (definite || g.cur_f == MS_HF_READ) ? MS_H_FAIL : MS_H_INFO;
     } else if (g.cur_f == MS_HF_READ) {
-      value = vc.y;                                                        // read_ok: the size of the set
+      value = m.p0;                                                        // read_ok: the size of the set
     }
     gen_hist(p, st, now, round, e, g, g.ops, outcome, g.cur_f, err, value);
     g.waiting_for = 0;
@@ -663,27 +711,18 @@ __global__ void k_release(Params p) {
       if ((uint32_t)(pos - p.head_sh[o][dest]) >= ring_cap_of(p, dest)) {
         latch_error(st, E_RING_OVERFLOW, dest);
       } else {
-        uint4* dst = ring_slot(p, p.ring_sh[o], dest, pos);
-        st_v4(dst, a); st_v4(dst + 1, b); st_v4(dst + 2, c);
+        ring_put(p, p.ring_sh[o], ring_index(p, dest, pos), a, b, c);
       }
     }
   }
 }
 
 // ------------------------------------------------------------------ node programs
-// Fields of a delivered message the node programs look at (2nd and 3rd vector
-// of the 48-B record); re-read from the ring (L1 hit) in every phase.
+// Fields of a delivered message the node programs look at (from ring_load).
 struct MsgView {
   uint32_t src, msg_id, p0;
   uint32_t tf;   // type | flags << 16
 };
-
-__device__ __forceinline__ MsgView view_load(const uint4* rec) {
-  const uint4 b = rec[1], c = rec[2];
-  MsgView v;
-  v.src = b.x; v.msg_id = b.z; v.tf = c.x; v.p0 = c.y;
-  return v;
-}
 
 // vals[] bits
 constexpr uint32_t V_FRESH = 1u << 31;  // broadcast value unseen so far (after PC: first sight = new)
@@ -1469,7 +1508,7 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
       if (tid == 0) latch_error(st, E_WINDOW_OVERFLOW, e);
       n = 0;
     }
-    const uint4* myring = p.ring + ring_base(p, e) * 3;
+    const size_t my0 = ring_base(p, e);   // slot (head + i) & my_mask of the window is ring slot my0 + that
     const uint32_t my_mask = ring_cap_of(p, e) - 1u;
     const bool is_server = (kind == MS_KIND_SERVER);
     const bool bcast = !GS && is_server && p.workload == MS_W_BROADCAST;
@@ -1489,7 +1528,9 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
     __syncthreads();
 
     // PA1: one pass over the window in arrival order, loads 2 records deep: order keys,
-    //      partition check at dequeue (net.clj:234), compact message class
+    //      partition check at dequeue (net.clj:234), compact message class.  A broadcast server's
+    //      window is nearly all compact gossip: it loads the keys first and a body only for a key
+    //      without kCompact.  Other endpoints never receive compact records: key and body together.
     {
       uint32_t err_val = 0xFFFFFFFFu;
       uint32_t snap_gone = 0xFFFFFFFFu;
@@ -1498,25 +1539,49 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
       const bool nb4 = nb_smem && deg <= 4;
       const uint32_t nr0 = (nb4 && deg > 0) ? s_nbr[0] : 0xFFFFFFFFu, nr1 = (nb4 && deg > 1) ? s_nbr[1] : 0xFFFFFFFFu;
       const uint32_t nr2 = (nb4 && deg > 2) ? s_nbr[2] : 0xFFFFFFFFu, nr3 = (nb4 && deg > 3) ? s_nbr[3] : 0xFFFFFFFFu;
+      const uint4* body = p.ring + p.ring_slots;
+      // with a latency or loss nearly every record is full (compact gossip needs both to be zero): load
+      // key and body together then, too, and still expand any compact key that is in the window
+      const bool keys_first = bcast && !need_rng && const_lat == 0;
       for (int base = 0; base < (int)n; base += 2 * nt) {
-        uint4 a[2], b[2], c[2];
+        uint4 a[2];
+        uint32_t q_src[2], q_tf[2], q_v[2], q_run[2];
 #pragma unroll
         for (int q = 0; q < 2; q++) {
           const int i = base + q * nt + tid;
           if (i < (int)n) {
-            const uint4* rp = myring + (size_t)((head + i) & my_mask) * 3;
-            a[q] = rp[0]; b[q] = rp[1]; c[q] = rp[2];
+            const size_t g = my0 + ((head + i) & my_mask);
+            a[q] = p.ring[g];
+            if (!keys_first) {
+              const uint4 b = body[2 * g], c = body[2 * g + 1];
+              q_src[q] = b.x; q_tf[q] = c.x; q_v[q] = c.y; q_run[q] = c.z;
+            }
+          }
+        }
+        if (bcast) {
+#pragma unroll
+          for (int q = 0; q < 2; q++) {
+            const int i = base + q * nt + tid;
+            if (i >= (int)n) continue;
+            if (a[q].y & kCompact) {
+              q_src[q] = (a[q].y & 0xFFFFFFu) - p.n_inj_tickets; q_tf[q] = MS_T_BROADCAST; q_v[q] = a[q].w; q_run[q] = 0;
+            } else if (keys_first) {
+              const size_t g = my0 + ((head + i) & my_mask);
+              const uint4 b = body[2 * g], c = body[2 * g + 1];
+              q_src[q] = b.x; q_tf[q] = c.x; q_v[q] = c.y; q_run[q] = c.z;
+            }
           }
         }
 #pragma unroll
         for (int q = 0; q < 2; q++) {
           const int i = base + q * nt + tid;
           if (i >= (int)n) continue;
-          const uint64_t rnd = (uint64_t)a[q].z | ((uint64_t)a[q].w << 32);
-          keyA[i] = (rnd << 24) | (uint64_t)(a[q].y & 0xFFFFFFu);
+          const uint32_t tk = a[q].y & 0xFFFFFFu;
+          const uint64_t rnd = (a[q].y & kCompact) ? compact_round(round, a[q].z) : ((uint64_t)a[q].z | ((uint64_t)a[q].w << 32));
+          keyA[i] = (rnd << 24) | (uint64_t)tk;
           keyB[i] = a[q].x;
-          const uint32_t src = b[q].x, tf = c[q].x, v = c[q].y;
-          if (a[q].y < p.n_inj_tickets && src < p.n_servers) inj_srv = true;   // injected on behalf of a server
+          const uint32_t src = q_src[q], tf = q_tf[q], v = q_v[q];
+          if (tk < p.n_inj_tickets && src < p.n_servers) inj_srv = true;   // injected on behalf of a server
           bool cut = false;
           if (np.pair_active && p.pair_bits)
             cut = (p.pair_bits[(size_t)e * p.pair_words + (src >> 5)] >> (src & 31)) & 1u;
@@ -1562,7 +1627,7 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
                 if (v >= p.n_values || v > V_MASK) err_val = v;
                 else val |= v;
               } else if (tc == GT_REPL_FULL) {                   // the snapshot row of (src, run p1)
-                const uint32_t run = c[q].z;
+                const uint32_t run = q_run[q];
                 const uint32_t rowi = src * p.gs_slots + (run & (p.gs_slots - 1));
                 if (src >= p.n_servers ||
                     __ldcg(p.gs_tag_sh[owner_of(src, p.n_servers, p.n_shards)] + rowi) != run) snap_gone = src;
@@ -1604,10 +1669,16 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
         const uint32_t e2 = t2 - p.n_inj_tickets;
         const uint32_t h2 = p.head[e2], n2 = p.limit[e2] - h2, cap2 = ring_cap_of(p, e2);
         if (n2 > 0 && n2 <= cap2) {
-          const uint4* base2 = p.ring + ring_base(p, e2) * 3;
+          // keys always; bodies unless e2 is a broadcast server that loads its keys first (PA1)
+          const size_t g2 = ring_base(p, e2);
           const uint32_t o2 = h2 & (cap2 - 1u), first = min(n2, cap2 - o2);
-          prefetch_l2_bulk(base2 + (size_t)o2 * 3, first * 48u);
-          if (n2 > first) prefetch_l2_bulk(base2, (n2 - first) * 48u);
+          prefetch_l2_bulk(p.ring + g2 + o2, first * 16u);
+          if (n2 > first) prefetch_l2_bulk(p.ring + g2, (n2 - first) * 16u);
+          if (GS || need_rng || const_lat != 0 || p.workload != MS_W_BROADCAST || p.kind[e2] != MS_KIND_SERVER) {
+            const uint4* body2 = p.ring + p.ring_slots + 2 * g2;
+            prefetch_l2_bulk(body2 + 2 * (size_t)o2, first * 32u);
+            if (n2 > first) prefetch_l2_bulk(body2, (n2 - first) * 32u);
+          }
         }
       }
     }
@@ -1775,10 +1846,10 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
           for (uint32_t pos = 0; pos < n; pos++) {
             const uint32_t i = ord[pos];
             if (!(vals[i] & V_RECV)) continue;
-            const uint4* rp = myring + (size_t)((head + i) & my_mask) * 3;
-            if (p.workload == MS_W_RAFT) rf_handle(c, rec_unpack(rp[0], rp[1], rp[2]));
-            else if (p.workload == MS_W_TXN_TREE) tt_handle(c, rec_unpack(rp[0], rp[1], rp[2]));
-            else txn_handle(c, rec_unpack(rp[0], rp[1], rp[2]));
+            const Rec m = ring_load(p, p.ring, my0 + ((head + i) & my_mask), round, e);
+            if (p.workload == MS_W_RAFT) rf_handle(c, m);
+            else if (p.workload == MS_W_TXN_TREE) tt_handle(c, m);
+            else txn_handle(c, m);
           }
           if (p.workload == MS_W_RAFT) { rf_actions(c); rf_note_busy(c); }
           if (p.workload == MS_W_TXN_TREE) tt_actions(c);
@@ -1792,7 +1863,7 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
       // ---- closed-loop client: replies in id order, timeout, at most one new request (gen_step)
       if (tid == 0) {
         Rec q;
-        const bool send = gen_step(p, st, e, now, round, myring, head, my_mask, n, ord, vals, q);
+        const bool send = gen_step(p, st, e, now, round, my0, head, my_mask, n, ord, vals, q);
         if (send) {
           s_gen[0] = make_uint4(q.src, q.dest, q.msg_id, q.in_reply_to);
           s_gen[1] = make_uint4(q.tf, q.p0, 0u, 0u);
@@ -1811,12 +1882,11 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
         uint32_t* skey = reinterpret_cast<uint32_t*>(tab);
         for (uint32_t pos = tid; pos < n; pos += nt) {
           const uint32_t i = ord[pos];
-          const uint4* rp = myring + (size_t)((head + i) & my_mask) * 3;
-          const uint4 vc = rp[2];
-          reg1[pos] = (uint64_t)vc.z | ((uint64_t)vc.w << 32);
-          skey[pos] = vc.y;
-          const uint32_t ty = vc.x & 0xFFFFu;                       // types the device does not know (>= 256) stay unknown
-          meta[i] = (uint16_t)((ty < 0xFFu ? ty : 0xFFu) | ((vc.x >> 8) & 0xFF00u));
+          const Rec m = ring_load_body(p, p.ring, my0 + ((head + i) & my_mask));
+          reg1[pos] = m.p1;
+          skey[pos] = m.p0;
+          const uint32_t ty = m.tf & 0xFFFFu;                       // types the device does not know (>= 256) stay unknown
+          meta[i] = (uint16_t)((ty < 0xFFu ? ty : 0xFFu) | ((m.tf >> 8) & 0xFF00u));
         }
         __syncthreads();
         if (tid == 0) {
@@ -1835,7 +1905,7 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
             q.p1 = reg1[pos];
             q.src = 0;
             if (svc == MS_SVC_SEQ_KV)                               // per-client view (service.clj:162-166)
-              q.src = (myring + (size_t)((head + i) & my_mask) * 3)[1].x;
+              q.src = ring_load_body(p, p.ring, my0 + ((head + i) & my_mask)).src;
             const bool keyed = q.type == MS_T_READ || q.type == MS_T_WRITE || q.type == MS_T_CAS;
             if (svc != MS_SVC_LIN_TSO && keyed && q.key >= p.sv_n_keys) { latch_error(st, E_VALUE_RANGE, q.key); continue; }
             if (svc != MS_SVC_LIN_TSO && !keyed) continue;   // no clause of the store's `case` matches: logged, no reply (service.clj:262-263)
@@ -2078,8 +2148,7 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
       const uint32_t mt = meta[i];
       const uint32_t sslot = mt & M_SRCSLOT;
       if (full_recv || !nb_smem || sslot == 0) {
-        const uint4* rp = myring + (size_t)((head + i) & my_mask) * 3;
-        Rec m = rec_unpack(rp[0], rp[1], rp[2]);
+        const Rec m = ring_load(p, p.ring, my0 + ((head + i) & my_mask), round, e);
         const uint64_t id = (use_blocks ? s_bbase[blk[pos]] : dense_base(p, st, m.round, m.ticket)) + m.idx;
         journal_raw(p, cx.chunk + k, id, true, m);
         const bool cl = cl_ep || (m.src >= p.n_servers && kind_is_client(p.kind[m.src]));
@@ -2184,11 +2253,11 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
           }
           fast = has_direct && !np.any_removed;
         } else {
-          const uint4* rp = myring + (size_t)((head + i) & my_mask) * 3;
-          const uint4 vb = rp[1], vc = rp[2];
+          const size_t g = my0 + ((head + i) & my_mask);
+          const Rec m = bcast ? ring_load(p, p.ring, g, round, e) : ring_load_body(p, p.ring, g);
           MsgView w;
-          w.src = vb.x; w.msg_id = vb.z; w.tf = vc.x; w.p0 = vc.y;
-          const uint64_t p1 = (uint64_t)vc.z | ((uint64_t)vc.w << 32);
+          w.src = m.src; w.msg_id = m.msg_id; w.tf = m.tf; w.p0 = m.p0;
+          const uint64_t p1 = m.p1;
           bool svc_emission = false;
           if constexpr (SV) {
             if (kind == MS_KIND_SERVICE) {
@@ -2218,13 +2287,13 @@ __global__ void __launch_bounds__(CLS == 3 ? 512 : 256, CLS == 3 ? 2 : MS_ROUND_
       }
       if (fast) {
         // server -> neighbor gossip into ring space this CTA already claimed: what emit_one does for it, without
-        // the general case's lookups (both ends are live servers, zero constant latency, no loss: agg_ok)
-        r.round = round; r.ticket = ticket; r.idx = j;                         // order key == id order (net.clj:197)
+        // the general case's lookups (both ends are live servers, zero constant latency, no loss: agg_ok);
+        // the record is compact, order key (round, ticket, j) == id order (net.clj:197)
         journal_raw(p, cx.chunk + n_recv + j, j, false, r);                    // net.clj:208
         cx.c_send_sv++;
         cx.c_zero++;
-        uint4* ring_o = p.ring_sh[owner_of(r.dest, p.n_servers, p.n_shards)];
-        rec_store(ring_o + ((size_t)r.dest * p.ring_cap_s + (direct & (p.ring_cap_s - 1u))) * 3, r);
+        ring_store_gossip(p.ring_sh[owner_of(r.dest, p.n_servers, p.n_shards)],
+                          (size_t)r.dest * p.ring_cap_s + (direct & (p.ring_cap_s - 1u)), j, ticket, round, r.p0);
       }
       if (__any_sync(FULL, valid && !fast)) emit_one(p, st, np, cx, valid && !fast, r, j, direct, has_direct);
     }
