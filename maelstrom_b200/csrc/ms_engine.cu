@@ -986,6 +986,31 @@ int ms_add_endpoint(ms_sim* s, const char* id, int kind) {
           (rc = s->dalloc(&P.sv_seq_vhas, K * kSeqHist)) || (rc = s->dalloc(&P.sv_seq_vcnt, K)))
         return rc;
       CK(cudaStreamSynchronize(s->stream));
+    } else {
+      // a service added again is a new one (service.clj:147-156, 290-296) and starts empty; the
+      // memsets go on the engine stream, ahead of the next round
+      Params& P = s->P;
+      const size_t K = P.sv_n_keys;
+      switch (svc) {
+        case MS_SVC_LIN_KV:
+          CK(cudaMemsetAsync(P.sv_lin_val, 0, K * sizeof(uint32_t), s->stream));
+          CK(cudaMemsetAsync(P.sv_lin_has, 0, K, s->stream));
+          break;
+        case MS_SVC_SEQ_KV:
+          CK(cudaMemsetAsync(P.sv_seq_vidx, 0, K * kSeqHist * sizeof(uint32_t), s->stream));
+          CK(cudaMemsetAsync(P.sv_seq_vval, 0, K * kSeqHist * sizeof(uint32_t), s->stream));
+          CK(cudaMemsetAsync(P.sv_seq_vhas, 0, K * kSeqHist, s->stream));
+          CK(cudaMemsetAsync(P.sv_seq_vcnt, 0, K * sizeof(uint32_t), s->stream));
+          CK(cudaMemsetAsync(P.sv_seq_cli, 0, (size_t)s->cfg.max_endpoints * sizeof(uint32_t), s->stream));
+          CK(cudaMemsetAsync(P.sv_scalars + 1, 0, sizeof(uint64_t), s->stream));
+          break;
+        case MS_SVC_LWW_KV:
+          CK(cudaMemsetAsync(P.sv_lww_val, 0, 2 * K * sizeof(uint32_t), s->stream));
+          CK(cudaMemsetAsync(P.sv_lww_has, 0, 2 * K, s->stream));
+          break;
+        default:
+          CK(cudaMemsetAsync(P.sv_scalars, 0, sizeof(uint64_t), s->stream));
+      }
     }
     s->P.sv_ep[svc] = idx;
     s->P.family |= 2u;   // from now on the round kernels with the service program compiled in
